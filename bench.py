@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          our CUDA path (libjsfe.so through the C ABI)
   python bench.py --impl reference ...                    the CPU restatement of the reference's path on the host cores
+  python bench.py ... --dump-outputs DIR                  also write the last timed step's results to DIR/*.npy
 
 One "step" = one pass of the whole hot path (pyramid -> FAST/NMS -> compaction -> angle+blur+rBRIEF for both eyes,
 then the left<->right Hamming + SAD stereo match) over a batch of `--pairs` synthetic stereo pairs per GPU.
@@ -224,6 +225,40 @@ def check_parity(cfg, pairs_seeds, get_pair, golden_dir, n_oracle=2):
         cmp(f"oracle seed{seed}", get_pair(i), dict(kps_l=kl, desc_l=dl, kps_r=kr, desc_r=dr, u_right=ur, depth=dp))
         checked += 1
     return checked, bad, notes
+
+
+DUMP_BYTES = 64 << 20
+
+
+def step_outputs(fe, n_pairs, stream):
+    """What the device-resident step hands its caller (jsfe_get_keypoints / jsfe_get_stereo), as float arrays for --dump-outputs:
+    the keypoint count of every slot and, for the pairs in `pairs` (all of them when they fit in DUMP_BYTES at full keypoint
+    capacity, else a sample fixed by seed 0 and the batch size), their results concatenated in pair order.  kps_* rows are
+    x, y, score, angle (degrees), octave, size."""
+    per_pair = fe.max_kp * (2 * (6 + 32) + 4) * 4         # two eyes' keypoints and descriptors, four stereo rows of the left eye
+    k = max(1, min(n_pairs, (DUMP_BYTES - 24 * n_pairs) // per_pair))
+    pairs = np.arange(n_pairs) if k == n_pairs else np.sort(np.random.default_rng(0).choice(n_pairs, k, replace=False))
+    chosen = set(pairs.tolist())
+    n = np.zeros(2 * n_pairs)
+    cols = {key: [] for key in ("kps_l", "desc_l", "kps_r", "desc_r", "u_right", "depth", "best_idx_r", "best_dist")}
+    for p in range(n_pairs):
+        kl, dl = fe.get_keypoints(2 * p, stream)
+        kr, dr = fe.get_keypoints(2 * p + 1, stream)
+        n[2 * p], n[2 * p + 1] = kl.shape[1], kr.shape[1]
+        if p not in chosen:
+            continue
+        for key, kps in (("kps_l", kl), ("kps_r", kr)):
+            f = kps.astype(np.float32)
+            f[3] = kps[3].view(np.float32)                    # the angle row holds float32 bits
+            cols[key].append(f)
+        cols["desc_l"].append(dl.astype(np.float32))
+        cols["desc_r"].append(dr.astype(np.float32))
+        for key, a in zip(("u_right", "depth", "best_idx_r", "best_dist"), fe.get_stereo(p, stream)):
+            cols[key].append(a.astype(np.float32))
+    out = {"n_keypoints": n, "pairs": pairs.astype(np.float64)}
+    for key, parts in cols.items():
+        out[key] = np.concatenate(parts, axis=1 if key.startswith("kps") else 0)
+    return out
 
 
 # ------------------------------------------------------------------------------------------------ CPU legs
@@ -574,6 +609,8 @@ def run_ours(args, cfg):
     launches = fe.launch_count() - l0
     clocks = sampler.stop()
     value = world * B * args.steps / (ms / 1e3)
+    # read before the e2e legs below reuse the handle's slots
+    outputs = step_outputs(fe, B, stream) if (rank == 0 and args.dump_outputs) else None
 
     # ---- parity of the timed configuration (device-resident results of the distinct pairs), asserted in this run
     parity = None
@@ -594,15 +631,14 @@ def run_ours(args, cfg):
     for _ in range(2):
         step_e2e()
     # the e2e call is synchronous (it returns with the results on the host), so its time is wall-clock, max over ranks
-    e2e_steps = max(3, min(args.steps, 50))
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         step_e2e()
     torch.cuda.synchronize()
     ms_e2e_serial = max_over_ranks((time.perf_counter() - t0) * 1e3)
     barrier()
-    e2e_serial = world * B * e2e_steps / (ms_e2e_serial / 1e3)
+    e2e_serial = world * B * args.steps / (ms_e2e_serial / 1e3)
     # two batches in flight (begin/end over two handles): every step still uploads its 2*B images and downloads its result slabs
     steps_e2e_overlapped(3)
     barrier()
@@ -856,7 +892,7 @@ def run_ours(args, cfg):
                     "step_ms": {"median": float(np.median(e2e_per_step)), "p95": float(np.percentile(e2e_per_step, 95)), "n": int(len(e2e_per_step))},
                     "how": "jsfe_process_host_pairs_begin/_end, two handles alternating (a batch uploads while the previous one computes); "
                            "pinned host images in, pinned host result slabs out, wall clock over all steps",
-                    "blocking_call": {"value": e2e_serial, "unit": UNIT, "ms_per_step": ms_e2e_serial / e2e_steps,
+                    "blocking_call": {"value": e2e_serial, "unit": UNIT, "ms_per_step": ms_e2e_serial / args.steps,
                                       "how": "one jsfe_process_host_pairs call per step (chunked 3-stream pipeline inside), nothing else in flight"},
                     "h2d_only_ms_per_step": h2d_ms, "h2d_only_gbs": 2 * B * cfg.height * cfg.width / h2d_ms / 1e6 if h2d_ms else None,
                     "host_input": "jsfe_host_alloc, " + ("cached pinned" if args.host_cached else "write-combined pinned")},
@@ -888,6 +924,10 @@ def run_ours(args, cfg):
                 line["adjacent"] = {"search_by_projection": sbp_microbench(), "remap_bilinear": remap_microbench()}
             except Exception as e:   # adjacent-row colour must never break the headline line
                 line["adjacent"] = {"search_by_projection": {"error": repr(e)[:200]}}
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -912,7 +952,13 @@ def main():
     ap.add_argument("--gather-transport", default="p2p", choices=["p2p", "nccl"], help="peer-memory stores over NVLink (CUDA IPC) or NCCL send/recv")
     ap.add_argument("--host-cached", action="store_true", help="input images in ordinary (cached) pinned memory instead of write-combined")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity check against goldens and oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed step computed in its last run (rank 0's pairs) to "
+                    "DIR/<name>.npy as float32 / float64, at most 64 MB; the inputs are seeded, so two builds compare output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's results; the reference arm keeps none")
     from jetson_slam_b200.configs import CONFIGS
     cfg = CONFIGS[args.workload]
     if args.impl == "reference":

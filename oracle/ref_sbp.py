@@ -1,8 +1,7 @@
 """ctypes binding of oracle/_ref/libsbpref.so: the reference's OWN host code of ORBmatcher::SearchByProjection(Frame&, const Frame&,
 th, bMono) (src/ORBmatcher.cpp:1647-1963) with Frame::AssignFeaturesToGrid / GetFeaturesInArea / PosInGrid (src/Frame.cpp:464-479,
 569-639, 696-706), cut out of the reference checkout at build time and compiled unmodified (oracle/ref_build/sbp_slice/).
-TEST INFRASTRUCTURE: used by tools/make_golden_sbp.py to produce tests/golden/sbpref_*.npz and, when the library is present, by the
-tests as a live cross-check.  Never imported by the product."""
+TEST INFRASTRUCTURE: used by tools/make_golden_sbp.py to produce tests/golden/sbpref_*.npz.  Never imported by the product."""
 from __future__ import annotations
 
 import ctypes as C

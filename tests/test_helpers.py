@@ -1,9 +1,14 @@
 """Adjacent rows (SURVEY.md 8f): the three stateless helper kernels of the tracking thread.
 CPU part: the oracle restatements against float64 math.  GPU part: the CUDA kernels (through the C ABI) bit-exact against
-the oracle AND against the reference's own kernels (oracle/_ref/libjsref.so, when it travelled to the box)."""
+the oracle AND against the outputs of the reference's own kernels on the same inputs (tests/golden/helpersref_scene3.npz, written
+by tools/make_golden_helpers.py on a B200)."""
+import os
+import zlib
+
 import numpy as np
 import pytest
 
+from conftest import ROOT
 from oracle import oracle as orc
 
 
@@ -22,6 +27,24 @@ def _scene(n=5000, seed=0):
 
 
 K = dict(fx=718.856, fy=718.856, cx=607.19, cy=185.2)
+BOX = dict(min_x=0.0, max_x=1241.0, min_y=0.0, max_y=376.0)
+FRUSTUM = dict(min_x=0, max_x=1241, min_y=0, max_y=376, n_levels=8, log_scale_factor=float(np.log(np.float32(1.2))), view_cos_angle=0.5)
+GOLDEN_REF = os.path.join(ROOT, "tests", "golden", "helpersref_scene3.npz")
+
+
+def gpu_case():
+    """The inputs of the GPU test: a 20000-point scene and 50000 descriptor pairs."""
+    rng = np.random.default_rng(5)
+    dl, dr = rng.integers(0, 256, size=(3000, 32), dtype=np.uint8), rng.integers(0, 256, size=(3100, 32), dtype=np.uint8)
+    il, ir = rng.integers(0, 3000, size=50000).astype(np.int32), rng.integers(0, 3100, size=50000).astype(np.int32)
+    return _scene(20000, 3), (il, ir, dl, dr)
+
+
+def checksum(scene, ham):
+    h = 0
+    for a in (*scene, *ham):
+        h = zlib.crc32(np.ascontiguousarray(a).tobytes(), h)
+    return h
 
 
 def test_oracle_projection_matches_float64():
@@ -56,60 +79,37 @@ def test_oracle_in_frustum_flags_are_consistent():
 
 @pytest.mark.gpu
 def test_helpers_match_oracle_and_reference_kernels():
-    import ctypes as C
     import torch
     from jetson_slam_b200 import frontend
-    from oracle import ref
     dev = torch.device("cuda", 0)
-    P, Pn, R, t, Ow, maxd, ima, imi = _scene(20000, 3)
+    scene, (il, ir, dl, dr) = gpu_case()
+    P, Pn, R, t, Ow, maxd, ima, imi = scene
     tt = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
     dP, dPn, dR, dt_, dOw, dmd, dima, dimi = map(tt, (P, Pn, R, t, Ow, maxd, ima, imi))
-    box = dict(min_x=0.0, max_x=1241.0, min_y=0.0, max_y=376.0)
     # --- projection
-    got = [x.cpu().numpy() for x in frontend.project_points(dP, dR, dt_, **K, **box)]
-    want = orc.project_points(P, R, t, **K, **box)
-    for g, w in zip(got, want):
+    got = [x.cpu().numpy() for x in frontend.project_points(dP, dR, dt_, **K, **BOX)]
+    want_proj = orc.project_points(P, R, t, **K, **BOX)
+    for g, w in zip(got, want_proj):
         assert np.array_equal(g.view(np.uint8), w.view(np.uint8))
     # --- Hamming pairs
-    rng = np.random.default_rng(5)
-    dl, dr = rng.integers(0, 256, size=(3000, 32), dtype=np.uint8), rng.integers(0, 256, size=(3100, 32), dtype=np.uint8)
-    il, ir = rng.integers(0, 3000, size=50000).astype(np.int32), rng.integers(0, 3100, size=50000).astype(np.int32)
     d = frontend.hamming_pairs(tt(il), tt(ir), tt(dl), tt(dr)).cpu().numpy()
     assert np.array_equal(d, orc.hamming_pairs(il, ir, dl, dr))
     # --- frustum
-    fr = dict(min_x=0, max_x=1241, min_y=0, max_y=376, n_levels=8, log_scale_factor=float(np.log(np.float32(1.2))), view_cos_angle=0.5)
-    got = [x.cpu().numpy() for x in frontend.in_frustum(dP, dPn, dmd, dima, dimi, dR, dt_, dOw, **K, **fr)]
-    want = orc.in_frustum(P, Pn, maxd, ima, imi, R, t, Ow, **K, **fr)
+    got = [x.cpu().numpy() for x in frontend.in_frustum(dP, dPn, dmd, dima, dimi, dR, dt_, dOw, **K, **FRUSTUM)]
+    want = orc.in_frustum(P, Pn, maxd, ima, imi, R, t, Ow, **K, **FRUSTUM)
     m = want[5] == 1
     assert np.array_equal(got[5], want[5]) and m.sum() > 100
     for g, w in zip(got[:5], want[:5]):
         assert np.array_equal(g[m].view(np.uint8), w[m].view(np.uint8))
-    # --- the reference's own kernels, when the prebuilt library is present
-    if ref.available():
-        L = ref.lib()
-        p = lambda x: C.c_void_p(x.data_ptr())
-        n = P.shape[1]
-        u, v, iz = (torch.empty(n, device=dev) for _ in range(3))
-        ok = torch.empty(n, dtype=torch.uint8, device=dev)
-        L.jsref_project_points(n, p(dP[0]), p(dP[1]), p(dP[2]), p(dR), p(dt_), K["fx"], K["fy"], K["cx"], K["cy"], 0.0, 1241.0, 0.0,
-                               376.0, p(u), p(v), p(iz), p(ok))
-        w = orc.project_points(P, R, t, **K, **box)
-        for g, ww in zip((u, v, iz, ok), w):
-            assert np.array_equal(g.cpu().numpy().view(np.uint8), ww.view(np.uint8)), "reference projection kernel != oracle"
-        iz2, u2, v2, vc2 = (torch.zeros(n, device=dev) for _ in range(4))
-        lv2 = torch.zeros(n, dtype=torch.int32, device=dev)
-        ok2 = torch.empty(n, dtype=torch.uint8, device=dev)
-        L.jsref_in_frustum(n, p(dP[0]), p(dP[1]), p(dP[2]), p(dPn[0]), p(dPn[1]), p(dPn[2]), p(dmd), p(dima), p(dimi), p(dR), p(dt_),
-                           p(dOw), K["fx"], K["fy"], K["cx"], K["cy"], 0, 1241, 0, 376, 8, fr["log_scale_factor"], 0.5, p(iz2), p(u2),
-                           p(v2), p(lv2), p(vc2), p(ok2))
-        assert np.array_equal(ok2.cpu().numpy(), want[5]), "reference frustum kernel != oracle"
-        for g, ww in zip((iz2, u2, v2, lv2, vc2), want[:5]):
-            assert np.array_equal(g.cpu().numpy()[m].view(np.uint8), ww[m].view(np.uint8)), "reference frustum outputs != oracle"
-        d2 = torch.empty(50000, dtype=torch.int32, device=dev)
-        t_il, t_ir, t_dl, t_dr = tt(il), tt(ir), tt(dl), tt(dr)   # keep the device buffers alive across the call
-        L.jsref_hamming_pairs(50000, p(t_il), p(t_ir), p(t_dl), p(t_dr), p(d2))
-        torch.cuda.synchronize()
-        assert np.array_equal(d2.cpu().numpy(), d)
+    # --- the reference's own kernels on the same inputs (their stored outputs)
+    ref = np.load(GOLDEN_REF)
+    assert int(ref["input_checksum"]) == checksum(scene, (il, ir, dl, dr)), "the seeded inputs changed: regenerate with tools/make_golden_helpers.py"
+    for k, w in zip(("proj_u", "proj_v", "proj_iz", "proj_ok"), want_proj):
+        assert np.array_equal(ref[k].view(np.uint8), w.view(np.uint8)), f"reference projection kernel != oracle ({k})"
+    assert np.array_equal(ref["frustum_ok"], want[5]), "reference frustum kernel != oracle"
+    for k, w in zip(("frustum_iz", "frustum_u", "frustum_v", "frustum_level", "frustum_view_cos"), want[:5]):
+        assert np.array_equal(ref[k].view(np.uint8), w[m].view(np.uint8)), f"reference frustum outputs != oracle ({k})"
+    assert np.array_equal(ref["hamming"], d)
 
 
 @pytest.mark.gpu

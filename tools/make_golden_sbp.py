@@ -19,7 +19,7 @@ from oracle import ref_sbp  # noqa: E402
 def main():
     if not ref_sbp.available():
         raise SystemExit("oracle/_ref/libsbpref.so is missing: make -C oracle/ref_build sbp")
-    for name in sbp_cases.CASES:
+    for name in [*sbp_cases.CASES, *sbp_cases.MORE_CASES]:
         c = sbp_cases.build(name)
         r = ref_sbp.search_by_projection(c["frame_last"], c["frame_cur"], c["pose_last"], c["pose_cur"], **c["camera"], th=c["th"],
                                          scale_factors=sbp_cases.SF, mono=c["mono"], check_orientation=c["check_orientation"])
